@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the RTI-MPC hot path (BASELINE.json: "A1 centroidal MPC solves/sec").
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--config NAME]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--config NAME] [--dump-outputs DIR]
 
 A "step" is one real-time-iteration solve (MPC::GetRealTimeUpdate: horizon maintenance -> linearise -> assemble ->
 QP -> line search -> trajectory update) of every instance in the batch.  Workload at N=1: BASELINE config #2,
@@ -102,6 +102,25 @@ def ipm_algorithmic_flops(N, nu, nf, n_samples, iters, refined_iters):
     return 2 * ((iters + 1) * fact + iters * per_it + refined_iters * per_ref + start)
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(outputs, out_dir):
+    """Write every per-instance array as out_dir/<name>.npy in float64.  Above DUMP_LIMIT_BYTES the same fixed, seeded sample of
+    instances is kept from every array and its indices are written as sample_rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrs = {k: np.asarray(v, np.float64) for k, v in outputs.items()}
+    B = len(next(iter(arrs.values())))
+    row_bytes = sum(a[0].nbytes for a in arrs.values())
+    if B * row_bytes > DUMP_LIMIT_BYTES:
+        keep = (DUMP_LIMIT_BYTES - (1 << 16)) // (row_bytes + 8)   # 64 KB left for the .npy headers
+        rows = np.sort(np.random.default_rng(0).choice(B, keep, replace=False))
+        arrs = {k: a[rows] for k, a in arrs.items()}
+        arrs["sample_rows"] = rows.astype(np.float64)
+    for k, a in arrs.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def oracle_latency(cfg_name, solves):
     """Single-thread latency of the oracle's RTI solve on the nominal instance (ms): p50, p95."""
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
@@ -172,6 +191,8 @@ def main():
     ap.add_argument("--gait-opt", type=int, default=0, metavar="K",
                     help="BASELINE config #3: per step every instance does solve -> dH/dtheta -> contact-time LP -> line search over "
                          "K candidates (K + 1 RTI solves per instance and step); use with --config a1_gait_opt_config --batch 64")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rank 0) to DIR/<name>.npy, to compare two builds output for output")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", 0))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
@@ -189,6 +210,8 @@ def main():
                     f"{args.scenarios} closed-loop scenarios cut across {world} GPU(s), plant = node 1 of the solved trajectory")
 
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes what the CUDA path computed: use it with --impl ours")
         if rank != 0:
             return
         sample = args.cpu_sample or 8 * cores
@@ -230,7 +253,7 @@ def main():
         m.SetStateTrajectoryWarmStart(states)
         return m
 
-    def run_leg(cfg_name, mode, batch, steps, warmup, gait_k=0, scenarios=0, detail=False):
+    def run_leg(cfg_name, mode, batch, steps, warmup, gait_k=0, scenarios=0, detail=False, capture=False):
         """One timed leg.  mode: 'solve' (config #2: `batch` instances per GPU, weak scaling), 'gait' (config #3: per step solve
         + dH/dtheta + contact-time LP + line search over gait_k candidates) or 'closed_loop' (config #5: `scenarios`
         closed-loop scenarios cut across the ranks, strong scaling).  Device time with CUDA events on the launching stream,
@@ -249,6 +272,7 @@ def main():
         mpc = make_mpc(cfg_name, B, st)
         dt_plant = c["integrator_dt"]
         gait_stats = {"grad_ok": 0, "best_hist": np.zeros(max(gait_k, 1), np.int64)}
+        last_gait = {}
         n_max = 12 * (N + 1) + (args.max_spline_vars or 160)
         # the buffer the decision vectors come back into: page-locked, as a controller that reads them every tick would hold it
         z_pinned = torch.zeros((B, n_max), dtype=torch.float64).pin_memory()
@@ -260,6 +284,9 @@ def main():
             ls = mpc.LineSearch(st, t0, ee, lp["xk"], lp["step"], K=gait_k)
             gait_stats["grad_ok"] = int((g["status"] == 0).sum())
             gait_stats["best_hist"] += np.bincount(np.maximum(ls["best"], 0), minlength=gait_k)
+            last_gait.update(grad_status=g["status"], n_contacts=g["n_contacts"], dHdtheta=g["raw"], lp_step=lp["step"], lp_xk=lp["xk"],
+                             lp_new_times=lp["new_times"], lp_status=lp["status"], ls_best=ls["best"], ls_costs=ls["costs"],
+                             ls_quality=ls["quality"])
 
         snapshot = []
 
@@ -290,8 +317,13 @@ def main():
         ms_dev = mpc.event_elapsed_ms(0, 1)
         barrier()
         launches = mpc.launch_count() - l0
-        res = mpc.download()
+        res = mpc.download(z_out=z_host if capture else None)
         out = {"B": B, "N": N, "mpc": mpc, "res": res, "launches": launches, "sizes": mpc.sizes(0), "gait_stats": gait_stats}
+        # with capture: the results of the last timed step's solve (in gait mode read back after its gradient, LP and line search, which
+        # leave them in place) and its gait outputs, copied before the loops below reuse the buffers; z is [B][n_max], the columns past
+        # an instance's own size stay zero
+        if capture:
+            out["outputs"] = {k: np.array(v) for k, v in {**res, **last_gait}.items()}
 
         kms = None
         if detail:   # per-kernel device time (CUDA events around each launch) over another `steps` steps, for the roofline entry
@@ -345,7 +377,8 @@ def main():
     main_mode = "closed_loop" if args.closed_loop else ("gait" if args.gait_opt else "solve")
     sampler = ClockSampler(local_rank)
     sampler.start()
-    leg = run_leg(args.config, main_mode, args.batch, args.steps, args.warmup, gait_k=args.gait_opt, scenarios=args.scenarios, detail=True)
+    leg = run_leg(args.config, main_mode, args.batch, args.steps, args.warmup, gait_k=args.gait_opt, scenarios=args.scenarios, detail=True,
+                  capture=bool(args.dump_outputs))
     clocks = sampler.stop()
     mpc, res, sz, kms, B, N = leg["mpc"], leg["res"], leg["sizes"], leg["kernel_ms"], leg["B"], leg["N"]
 
@@ -451,6 +484,8 @@ def main():
                                         "not the reference binary, which needs Eigen / pinocchio / Clarabel (absent here)",
                                 "sample": f"{sample} instances of the same synthetic workload x 20 RTI solves (2 warm-up) on {cores} threads, {el:.1f} s",
                                 "latency_p50_ms": p50, "latency_p95_ms": p95}
+    if args.dump_outputs:
+        dump_outputs(leg["outputs"], args.dump_outputs)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -13,6 +13,8 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 ORACLE_SO = os.path.join(_HERE, "liboracle.so")
 REF_SPLINES_SO = os.path.join(_HERE, "_ref", "libref_splines.so")
 REF_MPC_SO = os.path.join(_HERE, "_ref", "libref_mpc.so")   # the reference's own MPC sources over stand-in headers (ref_shim/)
+# a checkout of the reference project (bilevel-gait-gen); optional, it is not part of this repository
+REF_DIR = os.environ.get("BGG_REFERENCE_DIR", "")
 
 FORCE, POSITION = 0, 1
 NO_DERIV, FULL_DERIV, EMPTY = 0, 1, 2
@@ -23,11 +25,11 @@ _ip = C.POINTER(C.c_int)
 
 
 def build(force=False):
-    """Compile the oracle (and oracle/_ref when /root/reference is present). Building the checker is not using it."""
+    """Compile the oracle (and oracle/_ref when BGG_REFERENCE_DIR names the reference's sources). Building the checker is not using it."""
     if force or not os.path.exists(ORACLE_SO):
         subprocess.check_call(["make", "-C", _HERE, "liboracle.so"], stdout=subprocess.DEVNULL)
-    if os.path.isdir("/root/reference/mpc/spline") and (force or not os.path.exists(REF_SPLINES_SO) or not os.path.exists(REF_MPC_SO)):
-        subprocess.check_call(["make", "-C", _HERE, "ref"], stdout=subprocess.DEVNULL)
+    if REF_DIR and os.path.isdir(os.path.join(REF_DIR, "mpc", "spline")) and (force or not os.path.exists(REF_SPLINES_SO) or not os.path.exists(REF_MPC_SO)):
+        subprocess.check_call(["make", "-C", _HERE, "ref", "REF=" + os.path.abspath(REF_DIR)], stdout=subprocess.DEVNULL)
 
 
 def _dptr(a):

@@ -15,7 +15,7 @@ def pytest_configure(config):
 
 @pytest.fixture(scope="session", autouse=True)
 def _build_oracle():
-    """The oracle is test infrastructure: build it (and oracle/_ref when /root/reference exists) once per session."""
+    """The oracle is test infrastructure: build it (and oracle/_ref when BGG_REFERENCE_DIR names the reference's sources) once per session."""
     import pyoracle
     pyoracle.build()
     yield

@@ -169,19 +169,25 @@ def test_sparse_qp_export_matches_reference_assembly(cfg_name):
     gpu = common.make_gpu(cfg_name, B, states)
     gpu.GetRealTimeUpdate(states, t0, ee)
     qps = gpu.GetQPData(0, B)
+    import hashlib
     import pyoracle as po
+    digest = hashlib.sha256()   # the reference's QPs, against tests/golden/reference_outputs.json
     for b in range(B):
         o = common.make_oracle(cfg_name, states[b])
         o.assemble(states[b], 0.0, ee[b])
         _assert_same_qp(qps[b], o.qp())
-        if po.have_ref_mpc():
+        if not po.have_ref_mpc():
+            common._feed(digest, o.qp())   # the restatement's assembly is the reference's bit for bit (test_oracle_vs_reference_mpc.py)
+        else:
             # ... and against the reference's OWN assembly code (oracle/_ref/libref_mpc.so: mpc_single_rigid_body.cpp, mpc.cpp,
-            # qp_data.cpp, sparse_matrix_builder.cpp compiled from /root/reference; travels to the GPU box prebuilt)
+            # qp_data.cpp, sparse_matrix_builder.cpp compiled from BGG_REFERENCE_DIR when it is set)
             r = po.SrbMpc(cfg["num_nodes"], cfg["integrator_dt"], wl.robot(), which="ref", **wl.mpc_kwargs(cfg))
             r.set_costs(wl.target_tangent(cfg), np.asarray(cfg["Q"], float))
             r.set_warm_states(np.tile(states[b], (cfg["num_nodes"] + 1, 1)))
             r.solve(states[b], 0.0, ee[b])
+            common._feed(digest, r.qp())
             _assert_same_qp(qps[b], r.qp())
+    common.check_golden_reference(f"sparse_qp/{cfg_name}", digest)
 
 
 def test_receding_horizon_with_mirrored_trajectory():

@@ -16,7 +16,12 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PKG = os.path.join(ROOT, "bilevel-gait-gen_b200")
 SHIM_SO = os.path.join(PKG, "libmpc_b200.so")
 TEST_BIN = os.path.join(ROOT, "tests", "cpp", "test_shim")
-A1_URDF = "/root/reference/models/a1_description/urdf/a1.urdf"
+# a trimmed A1 model with the reference's joint tree and the fixture's constants, and the three configurations in the reference's
+# YAML layout; BGG_REFERENCE_DIR (a checkout of the reference project) substitutes the reference's own files
+REF_DIR = os.environ.get("BGG_REFERENCE_DIR", "")
+A1_URDF = (os.path.join(REF_DIR, "models", "a1_description", "urdf", "a1.urdf") if REF_DIR else
+           os.path.join(ROOT, "tests", "golden", "a1_trimmed.urdf"))
+REF_APPS = os.path.join(REF_DIR, "apps") if REF_DIR else os.path.join(ROOT, "tests", "golden", "apps")
 
 
 def test_shim_library_loads_and_exports_the_urdf_entry_point():
@@ -26,7 +31,6 @@ def test_shim_library_loads_and_exports_the_urdf_entry_point():
     assert os.path.exists(TEST_BIN)
 
 
-@pytest.mark.skipif(not os.path.exists(A1_URDF), reason="the reference's URDF is only present in the build container")
 def test_urdf_reader_matches_the_robot_constants_fixture():
     import bgg_b200 as bg
     lib = C.CDLL(SHIM_SO)
@@ -39,7 +43,6 @@ def test_urdf_reader_matches_the_robot_constants_fixture():
     assert np.abs(np.array(rb.hip_xy[:]).reshape(4, 2) - np.array(gold["hip_offsets_xy"])).max() < 1e-12
 
 
-@pytest.mark.skipif(not os.path.exists(A1_URDF), reason="the reference's URDF is only present in the build container")
 def test_urdf_reader_extracts_the_leg_chains_of_the_fixture():
     """host/urdf_consts.cpp: LegKinematicsFromURDF (what the inverse kinematics needs of the model) against tests/golden."""
     lib = C.CDLL(SHIM_SO)
@@ -52,14 +55,13 @@ def test_urdf_reader_extracts_the_leg_chains_of_the_fixture():
     assert np.abs(np.array(kin[:]) - np.array(want)).max() < 1e-15
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/apps"), reason="the reference's YAML files are only present in the build container")
 @pytest.mark.parametrize("name", ["a1_configuration", "a1_gait_opt_config", "a1_config_distr_rejection"])
 def test_config_parser_reads_the_reference_yaml_and_pins_the_named_workloads(name):
     """utils::ConfigParser + the MPCInfo fill of test/mpc_test.cpp:46-83 on the reference's own configuration files; the
     values must be the ones bilevel-gait-gen_b200/workloads.py (bench.py, tests) carries for the same name."""
     lib = C.CDLL(SHIM_SO)
     out = (C.c_double * 47)()
-    assert lib.bgg_host_parse_config(f"/root/reference/apps/{name}.yaml".encode(), out) == 0
+    assert lib.bgg_host_parse_config(os.path.join(REF_APPS, name + ".yaml").encode(), out) == 0
     v = list(out)
     cfg = wl.CONFIGS[name]
     assert int(v[0]) == cfg["num_nodes"]

@@ -3,14 +3,18 @@
 Every check of the reference's own test/splines_tests.cpp is restated here (known answers :66-105, coefficient
 reconstruction :109-158, add/remove polys :160-237, finite-difference partials :239-444) and run against
   * 'oracle' -- the restatement, always;
-  * 'ref'    -- the reference's own end_effector_splines.cpp compiled from /root/reference (oracle/_ref), when built.
-A third group compares restatement and compiled reference on seeded random splines, bit for bit.
+  * 'ref'    -- the reference's own end_effector_splines.cpp compiled from BGG_REFERENCE_DIR (oracle/_ref), when built.
+A third group compares restatement and compiled reference on seeded random splines, bit for bit; without the compiled
+reference, against the reference's values stored in tests/golden/reference_outputs.json (common.Recorded).
 """
 import math
+
+import hashlib
 
 import numpy as np
 import pytest
 
+import common
 import pyoracle as po
 from pyoracle import FORCE, POSITION
 
@@ -225,12 +229,17 @@ def test_coefficient_partials_fd(which):   # splines_tests.cpp:327-444
 
 
 # ---------------------------------------------------------------------------------------- restatement vs reference
-def _random_spline_pair(rng):
+def _ref_spline(times, sic, digest):
+    """The reference's compiled spline, or the restatement standing in for it; what it returns goes into `digest`."""
+    return common.Recorded(po.FootSpline(times, sic, 3, "ref" if po.have_ref() else "oracle"), digest)
+
+
+def _random_spline_pair(rng, digest):
     n = int(rng.integers(3, 8))
     gaps = rng.uniform(0.15, 0.45, size=n - 1)
     times = np.concatenate([[0.0], np.cumsum(gaps)])
     sic = bool(rng.integers(0, 2))
-    a, b = po.FootSpline(times, sic, 3, "oracle"), po.FootSpline(times, sic, 3, "ref")
+    a, b = po.FootSpline(times, sic, 3, "oracle"), _ref_spline(times, sic, digest)
     for _ in range(int(rng.integers(0, 3))):
         d = float(rng.uniform(0.2, 0.4))
         a.add_poly(d)
@@ -247,11 +256,11 @@ def _random_spline_pair(rng):
     return a, b
 
 
-@pytest.mark.skipif(not po.have_ref(), reason="oracle/_ref not built (reference sources absent)")
 def test_restatement_matches_compiled_reference_bitwise():
     rng = np.random.default_rng(0)
+    digest = hashlib.sha256()
     for trial in range(40):
-        a, b = _random_spline_pair(rng)
+        a, b = _random_spline_pair(rng, digest)
         if trial % 3 == 0:
             t_rm = float(rng.uniform(a.start_time(), 0.5 * a.end_time()))
             a.remove_poly(t_rm)
@@ -305,13 +314,14 @@ def test_restatement_matches_compiled_reference_bitwise():
         a.set_contact_times(ct2)
         b.set_contact_times(ct2)
         assert np.array_equal(a.times(), b.times())
+    common.check_golden_reference("splines_random", digest)
 
 
-@pytest.mark.skipif(not po.have_ref(), reason="oracle/_ref not built (reference sources absent)")
 def test_set_to_touchdown_matches_reference():
     times = [0, 0.3, 0.6, 0.9, 1.2]
+    digest = hashlib.sha256()
     for sic in (False, True):
-        a, b = po.FootSpline(times, sic, 3, "oracle"), po.FootSpline(times, sic, 3, "ref")
+        a, b = po.FootSpline(times, sic, 3, "oracle"), _ref_spline(times, sic, digest)
         td = a.next_td(0.05)
         assert td == b.next_td(0.05)
         a.set_to_touchdown(td - 0.04)
@@ -322,3 +332,4 @@ def test_set_to_touchdown_matches_reference():
                 a.set_to_touchdown(bad)
             with pytest.raises(po.OracleError):
                 b.set_to_touchdown(bad)
+    common.check_golden_reference("splines_set_to_touchdown", digest)

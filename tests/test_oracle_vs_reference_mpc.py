@@ -1,6 +1,6 @@
 """The oracle's restatement of the MPC hot path against the REFERENCE'S OWN SOURCES compiled here.
 
-oracle/_ref/libref_mpc.so (oracle/Makefile) is built from /root/reference/mpc/{trajectory, mpc, mpc_single_rigid_body,
+oracle/_ref/libref_mpc.so (oracle/Makefile) is built from $BGG_REFERENCE_DIR/mpc/{trajectory, mpc, mpc_single_rigid_body,
 rk_integrator, gait_optimizer}.cpp, mpc/models/{model, single_rigid_body_model}.cpp, mpc/qp/{qp_data, qp_interface,
 clarabel_interface}.cpp, mpc/spline/*.cpp and utils/sparse_matrix_builder.cpp -- unmodified -- over the stand-in headers of
 oracle/ref_shim/ (Eigen containers, pinocchio with injected robot constants, the Clarabel solver = the oracle's restatement
@@ -9,7 +9,13 @@ spline maintenance, linearisation, Euler discretisation, the six constraint emit
 stacking, status handling and foot-box adaptation, the merit line search, the trajectory update -- and the QP derivative
 chain of the gait optimiser.  These tests require the oracle to reproduce it BIT FOR BIT (SURVEY.md section 8 rows a5-a15)
 and the gait gradient to 1e-9 (a16-a19; the 1384 x 1384 differential system is factorised by two different LU codes).
+
+Where the reference's sources are absent (BGG_REFERENCE_DIR unset) every test runs against what the reference returned, stored in
+tests/golden/reference_outputs.json (common.Recorded: digests of the values in call order; the gait gradient as numbers).
 """
+import hashlib
+import os
+
 import numpy as np
 import pytest
 
@@ -17,15 +23,18 @@ import common
 from common import wl
 
 po = pytest.importorskip("pyoracle")
-pytestmark = pytest.mark.skipif(not po.have_ref_mpc(), reason="oracle/_ref/libref_mpc.so not built (needs /root/reference)")
+LIVE = po.have_ref_mpc()   # the reference's own sources compiled into oracle/_ref/libref_mpc.so
 
 
-def _make(cfg_name, which, state):
+def _make(cfg_name, which, state, digest=None):
+    """which "ref": the reference's compiled code, or the restatement standing in for it when that is absent; wrapped in
+    common.Recorded (sharing `digest`) so that what it returns is checked against the stored reference outputs."""
     cfg = wl.CONFIGS[cfg_name]
-    o = po.SrbMpc(cfg["num_nodes"], cfg["integrator_dt"], wl.robot(), which=which, **wl.mpc_kwargs(cfg))
+    src = "ref" if which == "ref" and LIVE else "oracle"
+    o = po.SrbMpc(cfg["num_nodes"], cfg["integrator_dt"], wl.robot(), which=src, **wl.mpc_kwargs(cfg))
     o.set_costs(wl.target_tangent(cfg), np.asarray(cfg["Q"], float))
     o.set_warm_states(np.tile(np.asarray(state, float), (cfg["num_nodes"] + 1, 1)))
-    return o
+    return common.Recorded(o, digest) if which == "ref" else o
 
 
 def _assert_same_qp_bitwise(r, o):
@@ -60,8 +69,9 @@ def test_rti_step_is_bitwise_the_reference(cfg_name):
     states[0] = cfg["srb_init"]
     ee[0] = wl.EE_NOMINAL
     seen = set()
+    digest = hashlib.sha256()
     for b in range(4):
-        r, o = _make(cfg_name, "ref", states[b]), _make(cfg_name, "oracle", states[b])
+        r, o = _make(cfg_name, "ref", states[b], digest), _make(cfg_name, "oracle", states[b])
         for _ in range(3):   # three RTI steps at t = 0 (the start of CreateInitialRun)
             sr = r.solve(states[b], 0.0, ee[b])
             so = o.solve(states[b], 0.0, ee[b])
@@ -70,6 +80,7 @@ def test_rti_step_is_bitwise_the_reference(cfg_name):
             _assert_same_qp_bitwise(r, o)
             _assert_same_step_bitwise(r, o)
     assert 0 in seen
+    common.check_golden_reference(f"rti_step/{cfg_name}", digest)
 
 
 def test_receding_horizon_is_bitwise_the_reference():
@@ -93,6 +104,7 @@ def test_receding_horizon_is_bitwise_the_reference():
         sizes.add((o.sizes()["n"], o.sizes()["m"]))
         state = o.states()[1].copy()
     assert len(sizes) > 1, "the horizon never changed size"
+    common.check_golden_reference("receding_horizon", r.digest)
 
 
 def test_infeasible_qp_takes_the_reference_path():
@@ -104,8 +116,9 @@ def test_infeasible_qp_takes_the_reference_path():
     states, _, ee = wl.batched_trot_inputs(cfg, 12, seed=0)
     ee[:, :, :2] += np.random.default_rng(5).uniform(-0.08, 0.08, (12, 4, 2))
     hit = 0
+    digest = hashlib.sha256()
     for b in range(12):
-        r, o = _make(cfg_name, "ref", states[b]), _make(cfg_name, "oracle", states[b])
+        r, o = _make(cfg_name, "ref", states[b], digest), _make(cfg_name, "oracle", states[b])
         st = [(r.solve(states[b], 0.0, ee[b]), o.solve(states[b], 0.0, ee[b])) for _ in range(3)]
         assert all(a == c for a, c in st), st
         _assert_same_qp_bitwise(r, o)
@@ -114,6 +127,7 @@ def test_infeasible_qp_takes_the_reference_path():
             hit += 1
             assert r.stats()["ee_box_x"] > cfg["ee_box_size"][0]
     assert hit >= 1, "no infeasible instance in this batch"
+    common.check_golden_reference("infeasible_qp", digest)
 
 
 @pytest.mark.parametrize("cfg_name", ["a1_configuration"])
@@ -129,12 +143,18 @@ def test_gait_gradient_matches_the_reference_chain(cfg_name):
     r, o = _make(cfg_name, "ref", init), _make(cfg_name, "oracle", init)
     assert r.initial_run(init, wl.EE_NOMINAL) == o.initial_run(init, wl.EE_NOMINAL) == 0
     assert r.solve(init, 0.0, wl.EE_NOMINAL) == o.solve(init, 0.0, wl.EE_NOMINAL) == 0
-    g_ref = r.gait_gradient()
-    assert g_ref is not None
     g_o = go.cost_gradient(o)
     n = len(g_o)
     assert n == sum(len(r.contact_times(e)[0]) for e in range(4))
-    assert np.abs(g_ref[:n] - g_o).max() <= 1e-9 * max(1.0, np.abs(g_o).max()), (g_ref[:n], g_o)
+    tol = 1e-9 * max(1.0, np.abs(g_o).max())
+    if LIVE:
+        g_live = r.gait_gradient()
+        assert g_live is not None
+        assert np.abs(g_live[:n] - g_o).max() <= tol, (g_live[:n], g_o)
+    if os.environ.get("BGG_RECORD_GOLDEN"):
+        common.check_golden_reference(f"gait_gradient/{cfg_name}", (g_live if LIVE else g_o)[:n].tolist())
+    g_ref = np.array(common.golden_reference(f"gait_gradient/{cfg_name}"))
+    assert len(g_ref) == n and np.abs(g_ref - g_o).max() <= tol, (g_ref, g_o)
 
 
 @pytest.mark.parametrize("cfg_name", ["a1_configuration", "a1_gait_opt_config"])
@@ -149,23 +169,44 @@ def test_contact_time_lp_is_the_one_the_reference_builds(cfg_name):
     init = np.asarray(cfg["srb_init"], float)
     r = _make(cfg_name, "ref", init)
     assert r.initial_run(init, wl.EE_NOMINAL) == 0 and r.solve(init, 0.0, wl.EE_NOMINAL) == 0
-    g = r.gait_gradient()
-    assert g is not None
     ct = [r.contact_times(e) for e in range(4)]
     n = sum(len(t) for t, _ in ct)
-    g = g[:n]
+    if LIVE:
+        g = r.gait_gradient()
+        assert g is not None
+        g = g[:n]
+    else:
+        if os.environ.get("BGG_RECORD_GOLDEN"):
+            common.check_golden_reference(f"gait_gradient/{cfg_name}", go.cost_gradient(r._obj).tolist())
+        g = np.array(common.golden_reference(f"gait_gradient/{cfg_name}"))
+        assert len(g) == n
+
+    def gait_lp(time, grad, solution=None):   # the reference's OptimizeContactTimes, or the restatement in its call shape
+        if LIVE:
+            out = r.gait_lp(time, grad, solution)
+        else:
+            A, lb, ub = go.gait_lp(ct, grad, time)
+            out = (2, A.toarray(), lb, ub, grad.copy())
+            if solution is not None:
+                xk_ = np.concatenate([t for t, _ in ct])
+                out = (0,) + out[1:] + (np.concatenate(go.contact_times_for(ct, xk_, solution, 1.0)),)
+        common._feed(r.digest, out)
+        return out
+
     for time in (0.0, 0.13):
         A_o, lb_o, ub_o = go.gait_lp(ct, g, time)
-        rc, A_r, lb_r, ub_r, q_r = r.gait_lp(time, g)
+        rc, A_r, lb_r, ub_r, q_r = gait_lp(time, g)
         assert rc == 2
         assert np.array_equal(A_r, A_o.toarray())
         assert np.array_equal(lb_r, lb_o) and np.array_equal(ub_r, ub_o) and np.array_equal(q_r, g)
     step = go.solve_gait_lp(ct, g, 0.0)
     xk = np.concatenate([t for t, _ in ct])
-    rc, _, _, _, _, new_times = r.gait_lp(0.0, g, step)
+    rc, _, _, _, _, new_times = gait_lp(0.0, g, step)
     assert rc == 0
     want = np.concatenate(go.contact_times_for(ct, xk, step, 1.0))
     assert np.array_equal(new_times, want), np.abs(new_times - want).max()
+    if not LIVE or os.environ.get("BGG_RECORD_GOLDEN"):   # with the live reference, its own gradient (1e-9 from the stored one) feeds the LP
+        common.check_golden_reference(f"contact_time_lp/{cfg_name}", r.digest)
 
 
 def test_adjust_for_current_contacts_is_the_references():
@@ -175,8 +216,9 @@ def test_adjust_for_current_contacts_is_the_references():
     cfg_name = "a1_configuration"
     cfg = wl.CONFIGS[cfg_name]
     init = np.asarray(cfg["srb_init"], float)
+    digest = hashlib.sha256()
     for early_by, expect_change in ((0.05, True), (0.15, False)):
-        r, o = _make(cfg_name, "ref", init), _make(cfg_name, "oracle", init)
+        r, o = _make(cfg_name, "ref", init, digest), _make(cfg_name, "oracle", init)
         assert r.initial_run(init, wl.EE_NOMINAL) == o.initial_run(init, wl.EE_NOMINAL) == 0
         before = [r.contact_times(e) for e in range(4)]
         swing = [e for e in range(4) if before[e][1][0] != po.TOUCH_DOWN][0]      # a foot that starts in swing
@@ -196,3 +238,4 @@ def test_adjust_for_current_contacts_is_the_references():
         assert r.solve(state, now, ee_now) == o.solve(state, now, ee_now)
         _assert_same_qp_bitwise(r, o)
         _assert_same_step_bitwise(r, o)
+    common.check_golden_reference("adjust_for_current_contacts", digest)

@@ -1,6 +1,7 @@
 """Developer diagnostic: config #5 (65 536 closed-loop scenarios, N = 50) tick by tick: solve and read-back time, iterations, QP size."""
-import sys, time, numpy as np, torch
-sys.path.insert(0, "/root/repo/tests"); sys.path.insert(0, "/root/repo/bilevel-gait-gen_b200")
+import os, sys, time, numpy as np, torch
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, os.path.join(ROOT, "tests")); sys.path.insert(0, os.path.join(ROOT, "bilevel-gait-gen_b200"))
 import common
 from common import wl
 c = wl.CONFIGS["a1_config_distr_rejection"]
