@@ -269,10 +269,14 @@ int bgg_create(const bgg_config* cfg, const bgg_robot* robot, bgg_handle** out) 
     h->device = cfg->device;
     Params& P = h->P;
     P.N = cfg->num_nodes;
-    P.max_nu = cfg->max_spline_vars > 0 ? cfg->max_spline_vars : 160;
+    P.max_nu = cfg->max_spline_vars > 0 ? cfg->max_spline_vars : kMaxSplineVars;
     if (P.max_nu < P.N + 1 || P.max_nu % 8) {
         delete h;
         return fail(BGG_EINVAL, "max_spline_vars must be a multiple of 8 and >= num_nodes + 1");
+    }
+    if (P.max_nu > kMaxSplineVars) {
+        delete h;
+        return fail(BGG_EINVAL, "max_spline_vars must not exceed 160: the condensing and KKT kernels are sized for at most 160 spline variables");
     }
     P.dt = cfg->integrator_dt;
     P.mass = robot->mass;

@@ -43,6 +43,8 @@ __device__ __forceinline__ double lds_c(unsigned addr) {
 // shared-memory load each (the A operand p_r Phi[r][i] is shared by a row's blocks).  The scalar 16 x 16 thread tiling
 // this replaces ran at 6 % of the FP64 peak (440 k cycles per instance for 1.8 MFMA, compiled without FMA contraction).
 constexpr int kCondAcc = 21;
+// the row pair p = 0 holds nb + 1 blocks; a block past kCondAcc would never be accumulated nor written
+static_assert((kMaxSplineVars + 7) / 8 + 1 <= kCondAcc, "k_condense: kCondAcc accumulators do not cover max_spline_vars = kMaxSplineVars");
 
 template <int NITEM>
 __global__ void __launch_bounds__(256, (NITEM == 1) ? 2 : 1) k_condense(Params P, WsLayout L, char* __restrict__ ws_base, int cap_nu, int want) {
@@ -208,7 +210,11 @@ __global__ void __launch_bounds__(256, (NITEM == 1) ? 2 : 1) k_condense(Params P
     }
     // full symmetric H to HBM (the IPM reads it column-wise, coalesced), straight from the accumulators: the block's
     // own entries and their mirror image; P_u (force weight on force variables, +1e-3 on everything: AddForceCost /
-    // AddDiagonalCost) goes on the diagonal
+    // AddDiagonalCost) goes on the diagonal.  Off the diagonal blocks H is exactly symmetric (one value, stored twice); inside
+    // a diagonal block (i, j) and (j, i) are two roundings of the same sum, (p_r Phi[r][i]) Phi[r][j] and
+    // (p_r Phi[r][j]) Phi[r][i], and may differ in the last bits.  Both are what the IPM consumes (the factorisation reads
+    // the lower triangle, the residuals H v both), so they are kept as they are: tests/test_gpu_linalg.py bounds each against
+    // the long-double sum.
 #pragma unroll
     for (int it = 0; it < NITEM; ++it)
 #pragma unroll

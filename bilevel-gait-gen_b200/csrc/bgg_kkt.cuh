@@ -42,6 +42,8 @@ struct KktView {
 };
 
 constexpr int kTileTab = 41 * 42 / 2;   // tiles of a 164 x 164 lower triangle (max_spline_vars 160 + padding)
+static_assert(kTileTab >= ((kMaxSplineVars + 3) / 4) * ((kMaxSplineVars + 3) / 4 + 1) / 2,
+              "kTileTab does not cover the 4 x 4 tiles of kMaxSplineVars force variables");
 
 // (ti << 8) | tl for t = 0 .. side (side + 1) / 2 - 1, tiles enumerated row by row
 __device__ inline void kkt_build_tile_table(uint16_t* tab, int side) {

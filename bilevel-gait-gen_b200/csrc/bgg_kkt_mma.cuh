@@ -54,6 +54,9 @@ struct KktWork {          // dense part: two row segments of K blocks for one wa
 };
 static_assert(sizeof(KktWork) == 8, "KktWork is read as two 32-bit words");
 constexpr int kMaxKktWork = 32;
+// row segments of at most kAccMax blocks that kkt_mma_setup lists for nb block rows (it drops any beyond kMaxKktWork)
+constexpr int kkt_segments(int nb) { return nb <= 0 ? 0 : kkt_segments(nb - 1) + (nb + kAccMax - 1) / kAccMax; }
+static_assert(kkt_segments((kMaxSplineVars + 7) / 8) <= kMaxKktWork, "kMaxKktWork does not cover the K blocks of kMaxSplineVars spline variables");
 
 // shared-memory accesses by 32-bit shared-window address: inside kkt_dense_mma nothing is a generic pointer, so the
 // compiler neither re-derives the window base per access nor has to assume that a store aliases its arguments

@@ -26,6 +26,10 @@ constexpr int kMaxStances = 4;       // stance segments per foot inside one hori
 constexpr int kEENodeStart = 4;      // EE_NODE_START, mpc_single_rigid_body.h:71
 constexpr int kNumForcePolys = 3;    // trajectory.cpp:33-34
 constexpr double kForceMult = 100.0; // end_effector_splines.h:152
+// Largest max_spline_vars (bgg_config) a handle accepts, and its default.  The register accumulators of k_condense
+// (kCondAcc), the KKT tile table (kTileTab) and the dense KKT work list (kMaxKktWork) are sized for it; bgg_create
+// refuses more.
+constexpr int kMaxSplineVars = 160;
 
 // knot / time types, numerically identical to the reference enums (spline_node.h:14-18, end_effector_splines.h:11-15)
 enum : uint8_t { kNoDeriv = 0, kFullDeriv = 1, kEmpty = 2 };

@@ -40,7 +40,9 @@ enum bgg_status {
  * (ClarabelInterface ctor, mpc/qp/clarabel_interface.cpp:18-27). */
 typedef struct bgg_config {
     int32_t num_nodes;        /* N, 4 < N <= 64 */
-    int32_t max_spline_vars;  /* cap on force+position spline variables per instance (0 = default 160) */
+    int32_t max_spline_vars;  /* cap on force+position spline variables per instance: a multiple of 8, >= num_nodes + 1 and
+                                 <= 160 (0 = default 160).  bgg_create refuses larger values: the condensing and KKT kernels
+                                 keep per-block tables sized for 160.  The shipped configurations need at most 148. */
     int32_t device;           /* CUDA device ordinal */
     int32_t ipm_max_iter;     /* 0 = default 50 */
     int32_t ipm_refine;       /* iterative refinement of the late solves against the regularised matrix: 0 / positive = one step (default), negative = none */
