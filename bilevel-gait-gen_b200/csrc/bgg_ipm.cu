@@ -27,6 +27,9 @@
 #include "bgg_kkt.cuh"
 #include "bgg_kkt_mma.cuh"
 #include "bgg_l2ops.cuh"
+#ifdef BGG_IPM_TRACE
+#include "bgg_ipm_trace.cuh"
+#endif
 
 namespace bgg {
 
@@ -41,6 +44,15 @@ __device__ long long g_ipm_prof[32];
 #define PROF_DECL
 #define PROF(k) do { } while (0)
 #define PROF_DUMP do { } while (0)
+#endif
+
+// Per-iteration trace (tests/test_gpu_ipm_trace.py): compiled in only with -DBGG_IPM_TRACE into a separate library
+// (tools/build_trace.sh), never into libbgg_b200.so.  csrc/bgg_ipm_trace.cuh describes the records.  TRACE(...) statements
+// run in the armed CTA only and add barriers there; without the macro they are empty.
+#ifdef BGG_IPM_TRACE
+#define TRACE(...) do { __VA_ARGS__ } while (0)
+#else
+#define TRACE(...) do { } while (0)
 #endif
 
 namespace {
@@ -414,6 +426,13 @@ __global__ void __launch_bounds__(kThreads, kThreads == 256 ? 2 : 1) k_ipm(Param
     }
     __syncthreads();
     PROF(0);
+#ifdef BGG_IPM_TRACE
+    const trace::Cfg tr_cfg = trace::g_cfg;
+    const bool tr_on = tr_cfg.buf != nullptr && tr_cfg.instance == b;
+    int tr_n = 0;
+    double* tr = nullptr;   // the current record, or nullptr
+    if (tr_on && tid == 0) ++trace::g_cfg.launches;
+#endif
 
     // ------------------------------------------------------------------------------------------------ operators
     IpmCtx ctx;
@@ -443,6 +462,11 @@ __global__ void __launch_bounds__(kThreads, kThreads == 256 ? 2 : 1) k_ipm(Param
         __syncthreads();
         kkt_assemble_mma(km);   // csrc/bgg_kkt_mma.cuh (also writes the identity padding)
         PROF(1);
+        TRACE(if (tr != nullptr) {
+            trace::put_vec(tr, trace::f_w, S.wv, m);
+            trace::put_vec(tr, trace::f_K, S.K, static_cast<int>(chol::doubles(nb)));
+            __syncthreads();
+        });
         chol::factor(S.K, nb, &s_flag);   // csrc/bgg_chol.cuh: DMMA block Cholesky, diagonal super-blocks inverted
         PROF(3);
         return s_flag == 0;
@@ -505,6 +529,21 @@ __global__ void __launch_bounds__(kThreads, kThreads == 256 ? 2 : 1) k_ipm(Param
     for (it = -1; it <= P.ipm_max_iter; ++it) {
         double uHu = 0, rt = 0, mu = 0;
         bool refine_now = false;
+        TRACE(if (tr_on) {
+            using namespace trace;
+            tr = begin_record(tr_cfg, tr_n++);
+            put(tr, f_it, it); put(tr, f_threads, kThreads); put(tr, f_spill, kSpill); put(tr, f_stage_phi, stage_phi);
+            put(tr, f_cap_nu, cap_nu); put(tr, f_cap_rows, cap_rows); put(tr, f_want, want); put(tr, f_confirm, confirm);
+            put(tr, f_N, N); put(tr, f_nu, nu); put(tr, f_nf, nf); put(tr, f_nb, nb); put(tr, f_ns, ns); put(tr, f_ne, ne);
+            put(tr, f_m, m); put(tr, f_neq, neq); put(tr, f_m_act, m_act);
+            put(tr, f_eps, eps); put(tr, f_delta, delta); put(tr, f_mu_f, mu_f); put(tr, f_tol_feas, P.ipm_tol_feas);
+            put(tr, f_tol_gap, P.ipm_tol_gap); put(tr, f_tol_infeas, P.ipm_tol_infeas); put(tr, f_nrm_q, nrm_q);
+            put(tr, f_nrm_d, nrm_d); put(tr, f_cost_const, cost_const); put(tr, f_tau, tau); put(tr, f_kap, kap);
+            put_vec(tr, f_u, S.u, nu); put_vec(tr, f_s, S.s, m); put_vec(tr, f_z, S.lam, m); put_vec(tr, f_y, S.nueq, neq);
+            if (tr != nullptr)
+                for (int i = tid; i < m; i += nth) tr[off(f_d) + i] = rhs_of(i);
+            __syncthreads();
+        });
         if (it >= 0) {
             // residuals  rx = H u + C'z + E'y + g tau ,  rz = C u + s - d tau ,  re = E u - e tau
             apply_H(S.u, S.Hu, false);
@@ -570,6 +609,14 @@ __global__ void __launch_bounds__(kThreads, kThreads == 256 ? 2 : 1) k_ipm(Param
             gap = n_gap;
             gscale = fmax(1.0, fmin(fabs(pc + cost_const), fabs(dc + cost_const)));   // full objective, as Clarabel's relative gap
             have_point = true;
+            TRACE(if (tr != nullptr) {
+                using namespace trace;
+                put(tr, f_fresh, fresh_rz); put(tr, f_mu, mu); put(tr, f_rt, rt); put(tr, f_uHu, uHu); put(tr, f_res_p, res_p);
+                put(tr, f_res_d, res_d); put(tr, f_gap, gap); put(tr, f_gscale, gscale); put(tr, f_bz, bz); put(tr, f_aty_n, aty_n);
+                put(tr, f_zn, zn); put(tr, f_pc, pc);
+                put_vec(tr, f_Hu, S.Hu, nu); put_vec(tr, f_rx, S.rd, nu); put_vec(tr, f_rz, S.rp, m); put_vec(tr, f_re, S.re, neq);
+                __syncthreads();
+            });
             if (res_d <= P.ipm_tol_feas * nrm_q && res_p <= P.ipm_tol_feas * nrm_d && gap <= P.ipm_tol_gap * gscale) {
                 if (fresh_rz) {
                     status = kSolved;
@@ -597,6 +644,7 @@ __global__ void __launch_bounds__(kThreads, kThreads == 256 ? 2 : 1) k_ipm(Param
             status = kOther;
             break;
         }
+        TRACE(trace::put(tr, trace::f_refine, refine_now););
 
         // Three solves with the one factorisation, one copy of the code: pass 0 the constant right-hand side (-g ; d ; e)
         // -> (x1, C x1, y1); pass 1 the affine step; pass 2 the combined step.  Row vectors while a pass runs: dl holds a2
@@ -638,6 +686,12 @@ __global__ void __launch_bounds__(kThreads, kThreads == 256 ? 2 : 1) k_ipm(Param
             apply_C(x, tslot, yx, 0.0);
             if (tid < neq) yx[tid] = (yx[tid] - S.a3[tid]) * inv_delta;
             __syncthreads();
+            TRACE(if (tr != nullptr && pass != 1) {
+                using namespace trace;
+                if (pass == 0) { put_vec(tr, f_x1, S.x1, nu); put_vec(tr, f_cx1, S.wv, m); put_vec(tr, f_y1, S.y1, neq); }
+                else { put_vec(tr, f_x2, S.du, nu); put_vec(tr, f_cx2, S.ds, m); put_vec(tr, f_a2, S.dl, m); put_vec(tr, f_y2, S.dnu, neq); }
+                __syncthreads();
+            });
             if (it < 0) break;
             // g'x, (H u)'x, d'z_x with z_x = W (C x - a2), e'y_x
             double r3[3] = {0, 0, 0};
@@ -712,8 +766,17 @@ __global__ void __launch_bounds__(kThreads, kThreads == 256 ? 2 : 1) k_ipm(Param
                 dkdt_aff = dkap * dtau;
             } else {
                 alpha = 0.99 * amax;
+                TRACE(trace::put(tr, trace::f_amax, amax););
             }
         }
+        TRACE(if (tr != nullptr && it >= 0 && !bad) {
+            using namespace trace;
+            put(tr, f_den, den); put(tr, f_sigma, sigma); put(tr, f_dkdt_aff, dkdt_aff); put(tr, f_dtau, dtau); put(tr, f_dkap, dkap);
+            put(tr, f_alpha, alpha);
+            put_vec(tr, f_du, S.du, nu); put_vec(tr, f_dz, S.dl, m); put_vec(tr, f_ds, S.ds, m); put_vec(tr, f_dy, S.dnu, neq);
+            put_vec(tr, f_drz, S.wv, m); put_vec(tr, f_dre, S.a3, neq);
+            __syncthreads();
+        });
         if (it < 0) {
             // starting point from the constant solve: u = x1, z = W (C x1 - d) with W = 1 / (1 + eps), s = -z, y = y1
             double mn[2] = {-1e300, -1e300};   // maxima of -s and -z = minus the minima
@@ -772,6 +835,7 @@ __global__ void __launch_bounds__(kThreads, kThreads == 256 ? 2 : 1) k_ipm(Param
     }
     if (it > P.ipm_max_iter) it = P.ipm_max_iter;
     if (it < 0) it = 0;
+    TRACE(trace::put(tr, trace::f_status_exit, status); trace::put(tr, trace::f_iters_exit, it); trace::put(tr, trace::f_refined_exit, n_refined););
 
     // ------------------------------------------------------------------------------------------------ outputs
     // the de-homogenised point (u, z, s, y) / tau; without a finite evaluation (have_point == false) u = 0 is written
@@ -836,5 +900,48 @@ extern "C" int bgg_debug_ipm_prof(long long* out32) {
     cudaMemcpyToSymbol(bgg::g_kkt_prof, zero, 8 * sizeof(long long));
     cudaMemcpyToSymbol(bgg::chol::g_chol_prof, zero, sizeof(zero));
     return rc;
+}
+#endif
+
+#ifdef BGG_IPM_TRACE
+// Arm the trace for the CTA of `instance` (its index in the launch's batch) with room for `cap` records; a negative instance
+// disarms it.  Every later launch of k_ipm in which that CTA iterates rewrites the records from the first.
+extern "C" int bgg_debug_ipm_trace_arm(int instance, int cap) {
+    using namespace bgg::trace;
+    Cfg c{};
+    if (cudaMemcpyFromSymbol(&c, g_cfg, sizeof c) != cudaSuccess) return 1;
+    if (c.buf != nullptr) cudaFree(c.buf);
+    c = Cfg{};
+    c.instance = -1;
+    if (instance >= 0 && cap > 0) {
+        if (cudaMalloc(&c.buf, sizeof(double) * kRecord * static_cast<size_t>(cap)) != cudaSuccess) return 2;
+        c.instance = instance;
+        c.cap = cap;
+    }
+    return cudaMemcpyToSymbol(g_cfg, &c, sizeof c) == cudaSuccess ? 0 : 3;
+}
+
+// hdr[0..5) = {doubles per record, fields, records written by the last traced launch, records stored, traced launches},
+// then (offset, length) per field; names: the field names, comma-separated.  With recs != nullptr also copies
+// min(stored, rec_cap) records.  Waits for the device.
+extern "C" int bgg_debug_ipm_trace_fetch(int* hdr, int hdr_cap, char* names, int names_cap, double* recs, int rec_cap) {
+    using namespace bgg::trace;
+    if (hdr_cap < 5 + 2 * kFields) return 1;
+    if (cudaDeviceSynchronize() != cudaSuccess) return 2;
+    Cfg c{};
+    if (cudaMemcpyFromSymbol(&c, g_cfg, sizeof c) != cudaSuccess) return 3;
+    const int stored = c.count < c.cap ? c.count : c.cap;
+    hdr[0] = kRecord; hdr[1] = kFields; hdr[2] = c.count; hdr[3] = stored; hdr[4] = c.launches;
+    for (int f = 0; f < kFields; ++f) { hdr[5 + 2 * f] = off(f); hdr[6 + 2 * f] = len_of(f); }
+#define BGG_TR_NAME(name, len) #name ","
+    static const char kNames[] = BGG_IPM_TRACE_FIELDS(BGG_TR_NAME);
+#undef BGG_TR_NAME
+    if (names_cap < static_cast<int>(sizeof kNames)) return 4;
+    for (size_t i = 0; i < sizeof kNames; ++i) names[i] = kNames[i];
+    if (recs != nullptr && stored > 0) {
+        const int n = stored < rec_cap ? stored : rec_cap;
+        if (cudaMemcpy(recs, c.buf, sizeof(double) * kRecord * static_cast<size_t>(n), cudaMemcpyDeviceToHost) != cudaSuccess) return 5;
+    }
+    return 0;
 }
 #endif
