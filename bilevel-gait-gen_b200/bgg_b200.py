@@ -75,6 +75,8 @@ def lib():
         L.bgg_solve_batch.argtypes = [C.c_void_p, _dp, _dp, _dp, _ip, _ip, _dp, _dp, _dp, C.c_int]
         L.bgg_qp_solve_batch.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _ip, _ip, _dp, _ip, _ip, _dp, _dp, _dp, C.POINTER(C.c_uint8),
                                          _dp, _dp, _dp, _ip, _ip]
+        L.bgg_qp_adjoint_batch.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _ip, _ip, _dp, _ip, _ip, _dp, C.POINTER(C.c_uint8),
+                                           _dp, _dp, _dp, _dp, _dp, _dp, _dp, _dp, _ip]
         L.bgg_controller_get_step.argtypes = [C.c_void_p, _dp, _dp, _dp]
         L.bgg_upload_inputs.argtypes = [C.c_void_p, _dp, _dp, _dp]
         L.bgg_solve_resident.argtypes = [C.c_void_p]
@@ -113,7 +115,7 @@ def lib():
 def exported_symbols():
     """Names include/bgg.h declares; used by the CPU-side ABI test."""
     return ["bgg_last_error", "bgg_device_count", "bgg_measure_fp64_peak", "bgg_create", "bgg_destroy", "bgg_set_costs", "bgg_batch_reset",
-            "bgg_set_warm_states", "bgg_set_contact_times", "bgg_solve_batch", "bgg_qp_solve_batch", "bgg_controller_tick_batch", "bgg_controller_get_step", "bgg_upload_inputs", "bgg_solve_resident",
+            "bgg_set_warm_states", "bgg_set_contact_times", "bgg_solve_batch", "bgg_qp_solve_batch", "bgg_qp_adjoint_batch", "bgg_controller_tick_batch", "bgg_controller_get_step", "bgg_upload_inputs", "bgg_solve_resident",
             "bgg_download_results", "bgg_synchronize", "bgg_advance_plant", "bgg_param_partials", "bgg_set_kinematics", "bgg_ik_batch", "bgg_targets_from_traj_batch", "bgg_set_profiling", "bgg_last_kernel_ms", "bgg_kernel_launch_count", "bgg_event_record", "bgg_event_elapsed_ms",
             "bgg_get_sizes", "bgg_get_dynamics", "bgg_get_condensed", "bgg_export_qp_csc", "bgg_gait_gradient_batch", "bgg_optimize_contact_times_batch",
             "bgg_line_search_batch", "bgg_get_adjoint",
@@ -259,10 +261,9 @@ class BatchedMPC:
     def solve_resident(self):
         self._chk(self.L.bgg_solve_resident(self.h))
 
-    def SolveQP(self, P, q, A, b, is_eq):
-        """QPInterface::SetupQP + Solve for a batch of QPs of one sparsity pattern (bgg_qp_solve_batch).  P, A: scipy sparse matrices
-        (values of the first QP) or lists of them (one per QP, same pattern); q [count][n], b [count][m]; is_eq [m].
-        Returns dict(x, y, s, status, iters)."""
+    @staticmethod
+    def _qp_pattern(P, A, is_eq):
+        """CSC pattern and stacked values of a batch of QPs (SolveQP / QPAdjoint): P, A scipy sparse matrices or lists of them."""
         import scipy.sparse as sp
         Ps = P if isinstance(P, (list, tuple)) else [P]
         As = A if isinstance(A, (list, tuple)) else [A]
@@ -270,19 +271,42 @@ class BatchedMPC:
         As = [sp.csc_matrix(a_, dtype=np.float64) for a_ in As]
         for m_ in Ps + As:
             m_.sort_indices()
-        count, n, m = len(Ps), Ps[0].shape[0], As[0].shape[0]
-        q = np.ascontiguousarray(np.asarray(q, np.float64).reshape(count, n))
-        b = np.ascontiguousarray(np.asarray(b, np.float64).reshape(count, m))
         pc, pr = np.ascontiguousarray(Ps[0].indptr, np.int32), np.ascontiguousarray(Ps[0].indices, np.int32)
         ac, ar = np.ascontiguousarray(As[0].indptr, np.int32), np.ascontiguousarray(As[0].indices, np.int32)
         pv = np.ascontiguousarray(np.stack([p_.data for p_ in Ps]))
         av = np.ascontiguousarray(np.stack([a_.data for a_ in As]))
         eq = np.ascontiguousarray(np.asarray(is_eq, np.uint8))
+        return len(Ps), Ps[0].shape[0], As[0].shape[0], pc, pr, pv, ac, ar, av, eq
+
+    def SolveQP(self, P, q, A, b, is_eq):
+        """QPInterface::SetupQP + Solve for a batch of QPs of one sparsity pattern (bgg_qp_solve_batch).  P, A: scipy sparse matrices
+        (values of the first QP) or lists of them (one per QP, same pattern); q [count][n], b [count][m]; is_eq [m].
+        Returns dict(x, y, s, status, iters)."""
+        count, n, m, pc, pr, pv, ac, ar, av, eq = self._qp_pattern(P, A, is_eq)
+        q = np.ascontiguousarray(np.asarray(q, np.float64).reshape(count, n))
+        b = np.ascontiguousarray(np.asarray(b, np.float64).reshape(count, m))
         x, y, s = np.zeros((count, n)), np.zeros((count, m)), np.zeros((count, m))
         st, it = np.zeros(count, np.int32), np.zeros(count, np.int32)
         self._chk(self.L.bgg_qp_solve_batch(self.h, count, n, m, _i(pc), _i(pr), _d(pv), _i(ac), _i(ar), _d(av), _d(q), _d(b),
                                             eq.ctypes.data_as(C.POINTER(C.c_uint8)), _d(x), _d(y), _d(s), _i(st), _i(it)))
         return dict(x=x, y=y, s=s, status=st, iters=it)
+
+    def QPAdjoint(self, P, A, is_eq, x, y, s, dx):
+        """ClarabelInterface::SetupDerivativeCalcs + CalcDerivativeWrtVecs / WrtMats for a batch of QPs of one sparsity pattern
+        (bgg_qp_adjoint_batch), at the points x [count][n], y / s [count][m] (normally what SolveQP returned) with loss gradient
+        dx [count][n].  P, A, is_eq as in SolveQP.  Returns dict(dz, dy, db [count][m] in the caller's row order, dA [count][nnz(A)] in
+        the order of A's sorted CSC data, status [count])."""
+        count, n, m, pc, pr, pv, ac, ar, av, eq = self._qp_pattern(P, A, is_eq)
+        x = np.ascontiguousarray(np.asarray(x, np.float64).reshape(count, n))
+        y = np.ascontiguousarray(np.asarray(y, np.float64).reshape(count, m))
+        s = np.ascontiguousarray(np.asarray(s, np.float64).reshape(count, m))
+        dx = np.ascontiguousarray(np.asarray(dx, np.float64).reshape(count, n))
+        dz, dy, db = np.zeros((count, n)), np.zeros((count, m)), np.zeros((count, m))
+        dA, st = np.zeros((count, len(ar))), np.zeros(count, np.int32)
+        self._chk(self.L.bgg_qp_adjoint_batch(self.h, count, n, m, _i(pc), _i(pr), _d(pv), _i(ac), _i(ar), _d(av),
+                                              eq.ctypes.data_as(C.POINTER(C.c_uint8)), _d(x), _d(y), _d(s), _d(dx), _d(dz), _d(dy),
+                                              _d(db), _d(dA), _i(st)))
+        return dict(dz=dz, dy=dy, db=db, dA=dA, status=st)
 
     def download(self, z_out=None):
         st, it = np.zeros(self.B, np.int32), np.zeros(self.B, np.int32)

@@ -215,7 +215,34 @@ int launch_qp_generic(int count, int n, int m, int mi, int me, int nnzP, int nnz
                       const int* Acol, const int* Arow, const double* Aval, const double* q, const double* b, const int* in_rows,
                       const int* eq_rows, const int* row_slot, double* ws, double* x, double* y, double* s, int32_t* status, int32_t* iters,
                       double tol_feas, double tol_gap, double tol_inf, double eps, double delta, int max_iter, int max_smem, cudaStream_t stream);
+constexpr int kQpAdjMaxDim_capi = 160;
+size_t qp_adj_ws_doubles(int n, int mi, int me);
+int launch_qp_adjoint(int count, int n, int m, int mi, int me, int nnzP, int nnzA, const int* Pcol, const int* Prow, const double* Pval,
+                      const int* Acol, const int* Arow, const double* Aval, const int* in_rows, const int* eq_rows, const int* row_slot,
+                      const double* x, const double* y, const double* s, const double* dx, double* ws, double* dz, double* dy, double* db,
+                      double* dA, int32_t* status, int max_smem, cudaStream_t stream);
 }  // namespace bgg
+
+// Row classification shared by bgg_qp_solve_batch and bgg_qp_adjoint_batch (csrc/bgg_qp_common.cuh): equality rows, and inequality
+// rows with at least one stored entry (an empty row reads 0 + s = b and is reported s = b, y = 0).  Returns an error message or null.
+struct QpRows {
+    std::vector<int> row_slot, in_rows, eq_rows;
+};
+static const char* qp_classify_rows(int m, int nnzA, const int32_t* A_rowidx, const uint8_t* is_eq, QpRows& R) {
+    std::vector<int> cnt(m, 0);
+    R.row_slot.assign(m, -1);
+    R.in_rows.clear();
+    R.eq_rows.clear();
+    for (int k = 0; k < nnzA; ++k) {
+        if (A_rowidx[k] < 0 || A_rowidx[k] >= m) return "row index out of range";
+        cnt[A_rowidx[k]]++;
+    }
+    for (int r = 0; r < m; ++r) {
+        if (is_eq[r]) { R.row_slot[r] = -(static_cast<int>(R.eq_rows.size()) + 2); R.eq_rows.push_back(r); }
+        else if (cnt[r] > 0) { R.row_slot[r] = static_cast<int>(R.in_rows.size()); R.in_rows.push_back(r); }
+    }
+    return nullptr;
+}
 
 extern "C" {
 
@@ -686,16 +713,9 @@ int bgg_qp_solve_batch(bgg_handle* h, int count, int n, int m, const int32_t* P_
     if (n > kQpMaxN_capi) return fail(BGG_EINVAL, "bgg_qp_solve_batch handles at most 128 variables (the MPC QP goes through bgg_solve_batch)");
     CU(cudaSetDevice(h->device));
     const int nnzP = P_colptr[n], nnzA = A_colptr[n];
-    // rows: equality rows, inequality rows with at least one stored entry (an empty row reads 0 + s = b and is reported s = b, y = 0)
-    std::vector<int> cnt(m, 0), row_slot(m, -1), in_rows, eq_rows;
-    for (int k = 0; k < nnzA; ++k) {
-        if (A_rowidx[k] < 0 || A_rowidx[k] >= m) return fail(BGG_EINVAL, "row index out of range");
-        cnt[A_rowidx[k]]++;
-    }
-    for (int r = 0; r < m; ++r) {
-        if (is_eq[r]) { row_slot[r] = -(static_cast<int>(eq_rows.size()) + 2); eq_rows.push_back(r); }
-        else if (cnt[r] > 0) { row_slot[r] = static_cast<int>(in_rows.size()); in_rows.push_back(r); }
-    }
+    QpRows R;
+    if (const char* err = qp_classify_rows(m, nnzA, A_rowidx, is_eq, R)) return fail(BGG_EINVAL, err);
+    const std::vector<int> &row_slot = R.row_slot, &in_rows = R.in_rows, &eq_rows = R.eq_rows;
     const int mi = static_cast<int>(in_rows.size()), me = static_cast<int>(eq_rows.size());
     const size_t wsd = qp_ws_doubles(n, mi, me);
     DevPool dev(h->stream);
@@ -729,6 +749,61 @@ int bgg_qp_solve_batch(bgg_handle* h, int count, int n, int m, const int32_t* P_
     if (s && m) CU(cudaMemcpyAsync(s, dsl, 8 * static_cast<size_t>(count) * m, cudaMemcpyDeviceToHost, st));
     if (status) CU(cudaMemcpyAsync(status, dst, 4 * static_cast<size_t>(count), cudaMemcpyDeviceToHost, st));
     if (iters) CU(cudaMemcpyAsync(iters, dit, 4 * static_cast<size_t>(count), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return BGG_OK;
+}
+
+int bgg_qp_adjoint_batch(bgg_handle* h, int count, int n, int m, const int32_t* P_colptr, const int32_t* P_rowidx, const double* P_val,
+                         const int32_t* A_colptr, const int32_t* A_rowidx, const double* A_val, const uint8_t* is_eq, const double* x,
+                         const double* y, const double* s, const double* dx, double* dz, double* dy, double* db, double* dA, int32_t* status) {
+    if (!h || count <= 0 || n <= 0 || m < 0 || !P_colptr || !P_rowidx || !P_val || !A_colptr || !A_rowidx || !A_val || !is_eq || !x || !dx ||
+        (m > 0 && (!y || !s)))
+        return fail(BGG_EINVAL, "null argument");
+    if (n > kQpMaxN_capi) return fail(BGG_EINVAL, "bgg_qp_adjoint_batch handles at most 128 variables, as bgg_qp_solve_batch");
+    CU(cudaSetDevice(h->device));
+    const int nnzP = P_colptr[n], nnzA = A_colptr[n];
+    QpRows R;
+    if (const char* err = qp_classify_rows(m, nnzA, A_rowidx, is_eq, R)) return fail(BGG_EINVAL, err);
+    const int mi = static_cast<int>(R.in_rows.size()), me = static_cast<int>(R.eq_rows.size());
+    if (n + me > kQpAdjMaxDim_capi)
+        return fail(BGG_EINVAL, "bgg_qp_adjoint_batch handles n + me <= 160 (variables plus equality rows; here " + std::to_string(n + me) +
+                                    "): the bordered system is factored in shared memory");
+    const size_t C = static_cast<size_t>(count), wsd = qp_adj_ws_doubles(n, mi, me);
+    DevPool dev(h->stream);
+    int *dPc = dev.get<int>(n + 1), *dPr = dev.get<int>(nnzP), *dAc = dev.get<int>(n + 1), *dAr = dev.get<int>(nnzA), *dIn = dev.get<int>(mi),
+        *dEq = dev.get<int>(me), *dSlot = dev.get<int>(m);
+    double *dPv = dev.get<double>(C * nnzP), *dAv = dev.get<double>(C * nnzA), *dxx = dev.get<double>(C * n), *dyy = dev.get<double>(C * m),
+           *dss = dev.get<double>(C * m), *ddx = dev.get<double>(C * n), *dws = dev.get<double>(C * wsd);
+    double *odz = dz ? dev.get<double>(C * n) : nullptr, *ody = (dy && m) ? dev.get<double>(C * m) : nullptr,
+           *odb = (db && m) ? dev.get<double>(C * m) : nullptr, *odA = (dA && nnzA) ? dev.get<double>(C * nnzA) : nullptr;
+    int32_t* dst = dev.get<int32_t>(C);
+    if (!dPc || !dPr || !dAc || !dAr || !dIn || !dEq || !dSlot || !dPv || !dAv || !dxx || !dyy || !dss || !ddx || !dws || !dst ||
+        (dz && !odz) || (dy && m && !ody) || (db && m && !odb) || (dA && nnzA && !odA))
+        return fail(BGG_ENOMEM, "device allocation failed");
+    cudaStream_t st = h->stream;
+    CU(cudaMemcpyAsync(dPc, P_colptr, 4 * (n + 1), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(dPr, P_rowidx, 4 * static_cast<size_t>(nnzP), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(dAc, A_colptr, 4 * (n + 1), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(dAr, A_rowidx, 4 * static_cast<size_t>(nnzA), cudaMemcpyHostToDevice, st));
+    if (mi) CU(cudaMemcpyAsync(dIn, R.in_rows.data(), 4 * static_cast<size_t>(mi), cudaMemcpyHostToDevice, st));
+    if (me) CU(cudaMemcpyAsync(dEq, R.eq_rows.data(), 4 * static_cast<size_t>(me), cudaMemcpyHostToDevice, st));
+    if (m) CU(cudaMemcpyAsync(dSlot, R.row_slot.data(), 4 * static_cast<size_t>(m), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(dPv, P_val, 8 * C * nnzP, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(dAv, A_val, 8 * C * nnzA, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(dxx, x, 8 * C * n, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(ddx, dx, 8 * C * n, cudaMemcpyHostToDevice, st));
+    if (m) CU(cudaMemcpyAsync(dyy, y, 8 * C * m, cudaMemcpyHostToDevice, st));
+    if (m) CU(cudaMemcpyAsync(dss, s, 8 * C * m, cudaMemcpyHostToDevice, st));
+    if (launch_qp_adjoint(count, n, m, mi, me, nnzP, nnzA, dPc, dPr, dPv, dAc, dAr, dAv, dIn, dEq, dSlot, dxx, dyy, dss, ddx, dws, odz, ody, odb,
+                          odA, dst, h->max_smem, st))
+        return fail(BGG_EINVAL, "the adjoint system needs more shared memory than the device offers");
+    h->launches += 1;
+    CU(cudaGetLastError());
+    if (dz) CU(cudaMemcpyAsync(dz, odz, 8 * C * n, cudaMemcpyDeviceToHost, st));
+    if (dy && m) CU(cudaMemcpyAsync(dy, ody, 8 * C * m, cudaMemcpyDeviceToHost, st));
+    if (db && m) CU(cudaMemcpyAsync(db, odb, 8 * C * m, cudaMemcpyDeviceToHost, st));
+    if (dA && nnzA) CU(cudaMemcpyAsync(dA, odA, 8 * C * nnzA, cudaMemcpyDeviceToHost, st));
+    if (status) CU(cudaMemcpyAsync(status, dst, 4 * C, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     return BGG_OK;
 }

@@ -10,6 +10,7 @@
 #include <cstdio>
 
 #include "bgg_kernels.cuh"
+#include "bgg_qp_common.cuh"
 
 namespace bgg {
 
@@ -63,22 +64,7 @@ __global__ void __launch_bounds__(256) k_qp_generic(QpDims D, const int* __restr
     __shared__ int s_flag;
 
     // ---- densify (values of this QP on the shared pattern)
-    for (size_t i = tid; i < static_cast<size_t>(mi + me) * n + static_cast<size_t>(n) * n; i += nth) ws[D.oA + i] = 0.0;
-    __syncthreads();
-    const double* Pv = Pval + static_cast<size_t>(b) * D.nnzP;
-    const double* Av = Aval + static_cast<size_t>(b) * D.nnzA;
-    for (int j = tid; j < n; j += nth) {
-        for (int k = Pcol[j]; k < Pcol[j + 1]; ++k) {   // a triangle or the full symmetric matrix: mirror, diagonal once
-            const int i = Prow[k];
-            Pd[static_cast<size_t>(i) * n + j] = Pv[k];
-            Pd[static_cast<size_t>(j) * n + i] = Pv[k];
-        }
-        for (int k = Acol[j]; k < Acol[j + 1]; ++k) {
-            const int slot = row_slot[Arow[k]];       // >= 0: inequality slot; < -1: equality slot -(slot + 2); -1: dropped row
-            if (slot >= 0) AI[static_cast<size_t>(slot) * n + j] = Av[k];
-            else if (slot < -1) AE[static_cast<size_t>(-(slot + 2)) * n + j] = Av[k];
-        }
-    }
+    qp_densify(n, mi, me, Pcol, Prow, Pval + static_cast<size_t>(b) * D.nnzP, Acol, Arow, Aval + static_cast<size_t>(b) * D.nnzA, row_slot, AI, AE, Pd);
     for (int r = tid; r < mi; r += nth) BI[r] = bb[in_rows[r]];
     for (int e = tid; e < me; e += nth) bE[e] = bb[eq_rows[e]];
     __syncthreads();

@@ -375,7 +375,9 @@ static bgg_handle* MakeSolverHandle() {   // the seam needs a device, a stream a
 ClarabelInterface::ClarabelInterface(const QPData& data, bool verbose) : QPInterface(data.num_decision_vars), h_(MakeSolverHandle()), verbose_(verbose) {}
 ClarabelInterface::ClarabelInterface(const ClarabelInterface& other)
     : QPInterface(other.num_decision_vars_), h_(MakeSolverHandle()), verbose_(other.verbose_), is_eq_(other.is_eq_),
-      solve_quality_(other.solve_quality_), dual_(other.dual_), primal_(other.primal_), slacks_(other.slacks_), dx_(other.dx_) {}
+      solve_quality_(other.solve_quality_), dual_(other.dual_), primal_(other.primal_), slacks_(other.slacks_), dx_(other.dx_),
+      have_solution_(other.have_solution_), have_derivative_(other.have_derivative_), d_x_(other.d_x_), d_y_(other.d_y_), d_dz_(other.d_dz_),
+      d_dy_(other.d_dy_), d_pattern_(other.d_pattern_), d_is_eq_(other.d_is_eq_) {}
 ClarabelInterface& ClarabelInterface::operator=(const ClarabelInterface& other) {
     if (this != &other) {
         num_decision_vars_ = other.num_decision_vars_;
@@ -386,6 +388,14 @@ ClarabelInterface& ClarabelInterface::operator=(const ClarabelInterface& other) 
         primal_ = other.primal_;
         slacks_ = other.slacks_;
         dx_ = other.dx_;
+        have_solution_ = other.have_solution_;
+        have_derivative_ = other.have_derivative_;
+        d_x_ = other.d_x_;
+        d_y_ = other.d_y_;
+        d_dz_ = other.d_dz_;
+        d_dy_ = other.d_dy_;
+        d_pattern_ = other.d_pattern_;
+        d_is_eq_ = other.d_is_eq_;
     }
     return *this;
 }
@@ -426,6 +436,8 @@ vector_t ClarabelInterface::Solve(const QPData& data) {
                              data.sparse_constraint_.outer.data(), data.sparse_constraint_.inner.data(), data.sparse_constraint_.values.data(),
                              data.cost_linear.data(), data.ub_.data(), is_eq_.data(), primal_.data(), dual_.data(), slacks_.data(), &status, &iters));
     solve_quality_ = static_cast<SolveQuality>(status);
+    have_solution_ = true;
+    have_derivative_ = false;
     if (solve_quality_ == PrimalInfeasible) {
         const std::string error = "Primal infeasible.";
         throw (error);   // what the caller catches (mpc_single_rigid_body.cpp:115-129)
@@ -439,6 +451,59 @@ vector_t ClarabelInterface::Computedx(const SparseCsc& P, const vector_t& q, con
     for (int j = 0; j < P.cols; ++j)
         for (int k = P.outer[j]; k < P.outer[j + 1]; ++k) dx_(P.inner[k]) += P.values[k] * xstar(j);
     return dx_;
+}
+
+void ClarabelInterface::SetupDerivativeCalcs(const vector_t& dx, double dl, double du, const QPData& data) {
+    if (dl != 0.0 || du != 0.0) throw std::runtime_error("ClarabelInterface::SetupDerivativeCalcs: dl and du are OSQP's bound terms and must be 0");
+    if (!have_solution_) throw std::runtime_error("ClarabelInterface::SetupDerivativeCalcs: no solution is held (call Solve first)");
+    const SparseCsc& A = data.sparse_constraint_;
+    const int n = A.cols, m = A.rows;
+    if (dx.size() != n || primal_.size() != n || dual_.size() != m || static_cast<int>(is_eq_.size()) != m)
+        throw std::runtime_error("ClarabelInterface::SetupDerivativeCalcs: the QP data does not match the last Solve");
+    d_dz_.resize(n);
+    d_dy_.resize(m);
+    int32_t status = 0;
+    Check(bgg_qp_adjoint_batch(h_, 1, n, m, data.sparse_cost_.outer.data(), data.sparse_cost_.inner.data(), data.sparse_cost_.values.data(),
+                               A.outer.data(), A.inner.data(), A.values.data(), is_eq_.data(), primal_.data(), dual_.data(), slacks_.data(),
+                               dx.data(), d_dz_.data(), d_dy_.data(), nullptr, nullptr, &status));
+    if (status != 0)
+        throw std::runtime_error(status == 1 ? "ClarabelInterface::SetupDerivativeCalcs: the differential system is singular"
+                                             : "ClarabelInterface::SetupDerivativeCalcs: a slack is not positive or an input is not finite");
+    d_x_ = primal_;
+    d_y_ = dual_;
+    d_pattern_ = A;
+    d_is_eq_ = is_eq_;
+    have_derivative_ = true;
+}
+
+void ClarabelInterface::CalcDerivativeWrtVecs(QPPartialsDense& partials) const {
+    if (!have_derivative_) throw std::runtime_error("ClarabelInterface::CalcDerivativeWrtVecs: SetupDerivativeCalcs has not run");
+    const int m = d_dy_.size();
+    int me = 0;
+    for (uint8_t e : d_is_eq_) me += e ? 1 : 0;
+    partials.dq = d_dz_;
+    partials.db = vector_t::Zero(me);
+    partials.dh = vector_t::Zero(m - me);
+    for (int r = 0, ie = 0, ii = 0; r < m; ++r) {
+        if (d_is_eq_[r]) partials.db(ie++) = -d_dy_(r);
+        else partials.dh(ii++) = -d_y_(r) * d_dy_(r);   // 0 on an inequality row without entries (dlam = 0 there)
+    }
+}
+
+void ClarabelInterface::CalcDerivativeWrtMats(QPPartialsDense& partials) const {
+    if (!have_derivative_) throw std::runtime_error("ClarabelInterface::CalcDerivativeWrtMats: SetupDerivativeCalcs has not run");
+    const int n = d_dz_.size(), m = d_dy_.size();
+    std::vector<int> idx(m);   // row -> row of dA (equality) or dG (inequality)
+    int me = 0, mi = 0;
+    for (int r = 0; r < m; ++r) idx[r] = d_is_eq_[r] ? me++ : mi++;
+    partials.dA = matrix_t::Zero(me, n);
+    partials.dG = matrix_t::Zero(mi, n);
+    for (int j = 0; j < n; ++j)
+        for (int k = d_pattern_.outer[j]; k < d_pattern_.outer[j + 1]; ++k) {
+            const int r = d_pattern_.inner[k];
+            if (d_is_eq_[r]) partials.dA(idx[r], j) = d_dy_(r) * d_x_(j) + d_y_(r) * d_dz_(j);
+            else partials.dG(idx[r], j) = d_y_(r) * d_dy_(r) * d_x_(j) + d_y_(r) * d_dz_(j);
+        }
 }
 
 bool MPC::ComputeDerivativeTerms() {

@@ -158,6 +158,21 @@ struct QPData {
     int GetTotalNumConstraints() const { return num_equality_ + num_inequality_; }
 };
 
+class MPC;
+// On the MPC's gait-optimisation path QPPartialsDense is a token (see the header comment) that records which MPC the derivative
+// terms belong to; ClarabelInterface::CalcDerivativeWrtVecs / WrtMats fill its matrices and vectors for a QP solved through the seam.
+struct QPPartialsDense {
+    const MPC* source = nullptr;
+    matrix_t dA, dG;
+    vector_t dq, db, dh;
+    void SetZero() {
+        dA.setZero();
+        dG.setZero();
+        dq.setZero();
+        db.setZero();
+        dh.setZero();
+    }
+};
 // The solver seam (mpc/include/qp/qp_interface.h:30-65) and its live implementation (mpc/include/qp/clarabel_interface.h:43-106,
 // mpc/qp/clarabel_interface.cpp:18-155), over bgg_qp_solve_batch: the interior-point kernel of the CUDA path on the QP it is handed.
 class QPInterface {
@@ -194,6 +209,17 @@ public:
     vector_t Computedx(const SparseCsc& P, const vector_t& q, const vector_t& xstar);   // dx = P x* + q (:604-612)
     vector_t Getdx() const { return dx_; }
     void SetVerbosity(bool verbose) { verbose_ = verbose; }
+    // The derivative of the last Solve's optimum (:262-602) over bgg_qp_adjoint_batch: the differential system at its primal, dual and
+    // slacks with right-hand side dx.  dl / du are OSQP's bound terms; on this path they must be zero, as the reference's call
+    // SetupDerivativeCalcs(dx, 0, 0, data) passes them (mpc.cpp:1047-1056).  Throws std::runtime_error if no solution is held or the
+    // system is singular; limits n <= 128 and n + (equality rows) <= 160.
+    void SetupDerivativeCalcs(const vector_t& dx, double dl, double du, const QPData& data);
+    // dq = dz, db = -dnu (equality rows), dh = -lam o dlam (inequality rows) (:182-196)
+    void CalcDerivativeWrtVecs(QPPartialsDense& partials) const;
+    // dA = dnu x' + nu dz' (equality rows x n), dG = D(lam) dlam x' + lam dz' (inequality rows x n), dense, on the pattern of the
+    // constraint matrix and zero elsewhere (:198-260).  Rows as SetupDerivativeCalcs numbers them: the equality rows in order, the
+    // inequality rows in order.
+    void CalcDerivativeWrtMats(QPPartialsDense& partials) const;
 
 private:
     bgg_handle* h_ = nullptr;
@@ -201,14 +227,13 @@ private:
     std::vector<uint8_t> is_eq_;
     SolveQuality solve_quality_ = Unsolved;
     vector_t dual_, primal_, slacks_, dx_;
+    bool have_solution_ = false, have_derivative_ = false;
+    // set by SetupDerivativeCalcs: the point, dz and dy (dlam / dnu in the caller's row order), the constraint pattern
+    vector_t d_x_, d_y_, d_dz_, d_dy_;
+    SparseCsc d_pattern_;
+    std::vector<uint8_t> d_is_eq_;
 };
 
-class MPC;
-// Tokens on the derivative path (see the header comment): they record which MPC the derivative terms belong to.
-struct QPPartialsDense {
-    const MPC* source = nullptr;
-    void SetZero() {}
-};
 struct QPPartials {   // mpc/include/qp/qp_partials.h:15-35
     const MPC* source = nullptr;
     int ee = -1, idx = -1;

@@ -140,6 +140,23 @@ int bgg_qp_solve_batch(bgg_handle* h, int count, int n, int m, const int32_t* P_
                        const int32_t* A_colptr, const int32_t* A_rowidx, const double* A_val, const double* q, const double* b,
                        const uint8_t* is_eq, double* x, double* y, double* s, int32_t* status, int32_t* iters);
 
+/* Derivative of the seam's QPs at a primal-dual point: ClarabelInterface::SetupDerivativeCalcs (mpc/qp/clarabel_interface.cpp:262-602)
+ * and the vectors CalcDerivativeWrtVecs / CalcDerivativeWrtMats form from it (:182-260), for `count` QPs on one pattern (the same
+ * conventions as bgg_qp_solve_batch).  With G the inequality rows of A, Ae the equality rows, lam = y on G's rows, nu = y on Ae's:
+ *     [ P    G'D(lam)   Ae' ] [dz  ]      [dx]
+ *     [ G    D(s)       0   ] [dlam]  = - [0 ]        (the reference's own +D(s) block)
+ *     [ Ae   0          0   ] [dnu ]      [0 ]
+ * x [count][n], y / s [count][m]: the point, in the caller's row order (normally what bgg_qp_solve_batch returned); dx [count][n]: the
+ * gradient of the loss in x (the reference passes P x + q, ClarabelInterface::Computedx :604-612).  Outputs, each may be NULL:
+ * dz [count][n] (= dq); dy [count][m] (dlam on inequality rows, dnu on equality rows); db [count][m] (-dnu on equality rows,
+ * dh = -lam o dlam on inequality rows); dA [count][nnz(A)] on A's pattern (dnu_r x_j + nu_r dz_j on an equality row r,
+ * lam_r dlam_r x_j + lam_r dz_j on an inequality row); status [count]: 0 ok, 1 a zero or non-finite pivot or a non-finite result,
+ * 2 s <= 0 on a kept inequality row or a non-finite input.  A QP of status 1 or 2 gets zero outputs.  Inequality rows without a stored
+ * entry are left out as in the solve (dlam = 0, dh = 0).  Limits: n <= 128 and n + (equality rows) <= 160, else BGG_EINVAL. */
+int bgg_qp_adjoint_batch(bgg_handle* h, int count, int n, int m, const int32_t* P_colptr, const int32_t* P_rowidx, const double* P_val,
+                         const int32_t* A_colptr, const int32_t* A_rowidx, const double* A_val, const uint8_t* is_eq, const double* x,
+                         const double* y, const double* s, const double* dx, double* dz, double* dy, double* db, double* dA, int32_t* status);
+
 /* The same solve split for measurement: copy inputs to HBM once, run the kernels on resident data, fetch results.
  * bgg_solve_resident returns with the solve enqueued on the handle's stream; it waits only for the step's first small kernel
  * (the per-instance set-up, whose sizes decide the shared-memory layout of the rest), not for the solve. */

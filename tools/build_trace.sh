@@ -12,5 +12,5 @@ OUT=${OUT:-$(pwd)/libbgg_b200_trace.so}
 OBJ=$(mktemp -d)
 trap 'rm -rf "$OBJ"' EXIT
 $NVCC $ARCH $COMMON -DBGG_IPM_TRACE -maxrregcount=128 -dc -o "$OBJ/bgg_ipm_trace.o" csrc/bgg_ipm.cu
-$NVCC $ARCH -shared -o "$OUT" build/bgg_prepare.o build/bgg_condense.o "$OBJ/bgg_ipm_trace.o" build/bgg_finish.o build/bgg_assemble.o build/bgg_gradient.o build/bgg_gait.o build/bgg_qp.o build/bgg_ik.o build/bgg_partials.o build/bgg_capi.o -lcudart
+$NVCC $ARCH -shared -o "$OUT" build/bgg_prepare.o build/bgg_condense.o "$OBJ/bgg_ipm_trace.o" build/bgg_finish.o build/bgg_assemble.o build/bgg_gradient.o build/bgg_gait.o build/bgg_qp.o build/bgg_qp_adjoint.o build/bgg_ik.o build/bgg_partials.o build/bgg_capi.o -lcudart
 echo "built $OUT"
