@@ -77,7 +77,9 @@ struct Smem {
 // What the operators below need.  They are force-inlined.  Measured on B200 (4096 solves): inlined 37.2 ms; as
 // __noinline__ functions (one copy of each in the binary: ncu shows the 0.4 MB kernel stalling on instruction fetch) with
 // the context by reference and every field copied to locals 41.1 ms, the same plus __isShared assumptions 39.2 ms,
-// context by value 83 ms -- the call boundary costs more than the instruction-cache misses it saves.
+// context by value 83 ms -- the call boundary costs more than the instruction-cache misses it saves.  Again with the
+// kernel body at 8.4 k instructions (B200, 1000 W, bench.py headline): inlined 28.6 ms; out of line with scalar arguments
+// and 32-bit shared-window addresses (one copy each, the body at 6.6 k instructions) 29.9 ms.
 struct IpmCtx {
     Smem S;
     const double* Hg;
@@ -110,7 +112,9 @@ static __device__ __forceinline__ void ipm_apply_C(const IpmCtx& c, const double
         for (int cc = 0; cc < 3; ++cc) {
             const double* vv = v + fbase[sp.ee] + cc * nfv[sp.ee] + sp.off;
             double s = 0;
-            for (int i = 0; i < sp.cnt; ++i) s += sp.w[i] * vv[i];
+            #pragma unroll
+            for (int i = 0; i < 4; ++i)   // cnt <= 4 (Sample::w): predicated, not a runtime-count loop unrolled with a remainder
+                if (i < sp.cnt) s += sp.w[i] * vv[i];
             fv[cc] = s;
         }
         double* o = out + 6 * j;
@@ -124,7 +128,9 @@ static __device__ __forceinline__ void ipm_apply_C(const IpmCtx& c, const double
     if (eout != nullptr && tid >= nth - 32 && tid - (nth - 32) < c.neq) {
         const EqRow& q = c.eq[tid - (nth - 32)];
         double s = -rhs_scale * q.rhs;
-        for (int i = 0; i < q.cnt; ++i) s += q.w[i] * v[q.col[i]];
+        #pragma unroll
+        for (int i = 0; i < 2; ++i)   // cnt <= 2 (EqRow::w)
+            if (i < q.cnt) s += q.w[i] * v[q.col[i]];
         eout[tid - (nth - 32)] = s;
     }
     __syncthreads();
@@ -133,7 +139,9 @@ static __device__ __forceinline__ void ipm_apply_C(const IpmCtx& c, const double
         const int cc = e & 1, foot = (e >> 1) & 3, kk = e >> 3, kf = kk * 4 + foot;
         const double* vv = v + nf + pbase[foot] + cc * npv[foot] + S.poff[kf];
         double s = -S.tkc[kk * 2 + cc];
-        for (int i = 0; i < S.pcnt[kf]; ++i) s += S.pw[2 * kf + i] * vv[i];
+        #pragma unroll
+        for (int i = 0; i < 2; ++i)   // pcnt <= 2
+            if (i < S.pcnt[kf]) s += S.pw[2 * kf + i] * vv[i];
         out[6 * ns + 2 * e] = s;
         out[6 * ns + 2 * e + 1] = -s;
     }
@@ -204,8 +212,9 @@ static __device__ __forceinline__ void ipm_add_Ct(const IpmCtx& c, const double*
                     for (int r = 0; r < c.neq; ++r) {
                         const EqRow& q = c.eq[r];
                         if (q.pad != grp) continue;
-                        for (int i = 0; i < q.cnt; ++i)
-                            if (q.col[i] == col) se += ey[r] * q.w[i];
+                        #pragma unroll
+                        for (int i = 0; i < 2; ++i)
+                            if (i < q.cnt && q.col[i] == col) se += ey[r] * q.w[i];
                     }
                     s += escale * se;
                 }
@@ -340,6 +349,7 @@ __global__ void __launch_bounds__(kThreads, kThreads == 256 ? 2 : 1) k_ipm(Param
         if (stage_phi) {
             S.phi = p;
             S.phi_stride = nf;
+            #pragma unroll 1
             for (int i = tid; i < nkc * nf; i += nth) p[i] = phipos[static_cast<size_t>(i / nf) * L.max_nu + (i % nf)];
         } else {
             S.phi = phipos;
@@ -374,6 +384,7 @@ __global__ void __launch_bounds__(kThreads, kThreads == 256 ? 2 : 1) k_ipm(Param
     if (tid == 0) {
         int e = 0;
         s_sb[0] = 0;
+        #pragma unroll 1
         for (int j = 0; j < ns; ++j)
             while (samples[j].ee > e) s_sb[++e] = j;
         while (e < kNumEE) s_sb[++e] = ns;
@@ -505,12 +516,14 @@ __global__ void __launch_bounds__(kThreads, kThreads == 256 ? 2 : 1) k_ipm(Param
     };
 
     double nrm_q = 1.0, nrm_d = 1.0;
+    #pragma unroll 1
     for (int r = 0; r < kNx; ++r) nrm_q = fmax(nrm_q, fmax(fabs(P.w[r]), fabs(P.Phi_w[r])));
     {
         double v = 0;
         #pragma unroll 1
         for (int i = tid; i < m; i += nth)
             if (S.lam[i] > 0.0) v = fmax(v, fabs(rhs_of(i)));
+        #pragma unroll 1
         for (int r = 0; r < neq; ++r) v = fmax(v, fabs(s_eq[r].rhs));
         nrm_d = fmax(1.0, block_reduce<kMax>(v, S.red));
     }
@@ -587,6 +600,7 @@ __global__ void __launch_bounds__(kThreads, kThreads == 256 ? 2 : 1) k_ipm(Param
             const double gu = r8[1];
             double ey = 0, n_re = 0;
             double yn = 0;
+            #pragma unroll 1
             for (int r = 0; r < neq; ++r) {
                 ey += s_eq[r].rhs * S.nueq[r];
                 n_re = fmax(n_re, fabs(S.re[r]));
@@ -710,6 +724,7 @@ __global__ void __launch_bounds__(kThreads, kThreads == 256 ? 2 : 1) k_ipm(Param
             block_reduce_multi<3, 0>(r3, S.red);
             PROF(13);
             double eyx = 0;
+            #pragma unroll 1
             for (int r = 0; r < neq; ++r) eyx += s_eq[r].rhs * yx[r];
             if (pass == 0) {
                 den = kap / tau - r3[0] - r3[2] - eyx + uHu / (tau * tau) - 2.0 * r3[1] / tau;
